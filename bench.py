@@ -53,6 +53,10 @@ def parse():
     ap.add_argument("--cpu-steps", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stock-torch", action="store_true", help="skip the stock-PyTorch-on-the-GPU leg (oracle step on cuda)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what one more step of the timed path computes from the initial weights "
+                         "(loss, metrics, depth maps, poses, a fixed sample of the updated parameters) as DIR/<name>.npy, "
+                         "float32: identical inputs from run to run, to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -372,6 +376,25 @@ def time_kernels(args, dev, pk):
     return res
 
 
+def dump_outputs(directory, out, model, max_elems=1 << 21):
+    """What a caller of the training step receives from a call: the loss, its metrics, the four inverse-depth maps, the two
+    context poses, and the updated parameters.  The parameters (130 M) and any array of more than `max_elems` elements are
+    stored as a fixed, seeded sample of `max_elems` of them, which bounds the files to about 40 MB."""
+    import numpy as np
+    arrays = {"loss": out["loss"], **out["metrics"]}
+    arrays.update({"inv_depth%d" % i: d for i, d in enumerate(out["inv_depths"])})
+    arrays.update({"pose%d" % j: p.mat for j, p in enumerate(out["poses"])})
+    arrays["parameters"] = torch.cat([p.detach().reshape(-1) for p in model.parameters()])
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > max_elems:
+            idx = torch.randint(t.numel(), (max_elems,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
+    log("outputs of the step from the initial state written to %s (%s)" % (directory, ", ".join(sorted(arrays))))
+
+
 def apply_variants(settings, PF, _lib, _losses):
     """--set KEY=0|1 overrides; returns the EFFECTIVE setting of every variant (library defaults where not overridden)."""
     setters = {"pack_fold": lambda v: PF.set_pack_fold(v), "loss_grouped": _losses.set_grouped_kernel,
@@ -435,6 +458,23 @@ def run_ours(args):
     hb = make_host_batch(B, H, W, rank)
     dbatch = to_device(hb, dev)
     state = {}
+    if args.dump_outputs:
+        # Two runs of the same steps drift apart (split-K partial sums land in any order, and Adam's first updates are
+        # +-lr for every gradient that is only rounding noise): the dumped step starts again from this initial state.
+        start = ([p.detach().clone() for p in model.parameters()], None if args.torch_adam else opt.state_dict())
+
+    def restore_start():
+        with torch.no_grad():
+            for p, v in zip(model.parameters(), start[0]):
+                p.copy_(v)
+        if args.torch_adam:
+            for st in opt.state.values():
+                for v in st.values():
+                    if torch.is_tensor(v):
+                        v.zero_()
+        else:
+            opt.load_state_dict(start[1])
+            opt.repack()            # the forward tiles of the stored weights (a replayed graph does not check them)
 
     def step(batch):
         zero_grad()
@@ -442,7 +482,7 @@ def run_ours(args):
         out["loss"].backward()
         reduce_grads()
         opt.step()
-        state["loss"] = out["loss"]
+        state["out"] = out
 
     def timed_region(fn, steps):
         if world > 1:
@@ -463,7 +503,7 @@ def run_ours(args):
         t_w = time.time()
         step(dbatch)
         torch.cuda.synchronize()
-        log("warm-up step %d: %.1f ms (loss %.5f)" % (i, (time.time() - t_w) * 1e3, float(state["loss"].item())))
+        log("warm-up step %d: %.1f ms (loss %.5f)" % (i, (time.time() - t_w) * 1e3, float(state["out"]["loss"].item())))
     eager_step = step
     graph_info = None
     graphs = None
@@ -490,7 +530,8 @@ def run_ours(args):
                     reduce_grads()
                     opt.step()
                 per_graph_launches = _lib.launch_count() - l0
-                graphs[fl] = (g, out["loss"])
+                # the loss module keeps ONE metrics dict, refilled by every call: hold this graph's own metric tensors
+                graphs[fl] = (g, dict(out, metrics=dict(out["metrics"])))
         except Exception as e:      # a failed capture is not sticky: fall back to eager enqueue and say so in the JSON line
             log("whole-step capture failed (%s): falling back to eager steps" % repr(e)[:300])
             graphs = None
@@ -506,14 +547,14 @@ def run_ours(args):
 
             def step(batch):
                 # `batch` must be the static device batch the graphs were captured on (dbatch); e2e copies into it
-                g, loss_t = graphs[random.random() < flip_prob]
+                g, out = graphs[random.random() < flip_prob]
                 g.replay()
-                state["loss"] = loss_t
+                state["out"] = out
 
         for _ in range(2):
             step(dbatch)
         torch.cuda.synchronize()
-        log("graph replay ok (loss %.5f)" % float(state["loss"].item()))
+        log("graph replay ok (loss %.5f)" % float(state["out"]["loss"].item()))
     # host time to ENQUEUE one step on an idle GPU (no sync inside): step time close to this = launch-bound
     torch.cuda.synchronize()
     t_q = time.perf_counter()
@@ -535,6 +576,14 @@ def run_ours(args):
     if graph_info is not None:
         launches = graph_info["library_launches_per_graph"] * args.steps     # replayed kernel nodes of our library
     log("timed region: %.1f ms/step (host CPU %.1f ms/step), %d library launches" % (ms / args.steps, cpu_ms, launches))
+    if args.dump_outputs:
+        # one more step of the timed path (the same graphs, or eager steps) from the initial weights and optimizer state
+        restore_start()
+        random.seed(42)             # the same left-right flip draw whatever ran before (graphs, eager steps, warm-up count)
+        step(dbatch)
+        torch.cuda.synchronize()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, state["out"], model)
 
     def e2e_step():
         if graph_info is not None:
@@ -546,7 +595,7 @@ def run_ours(args):
             step(dbatch)
         else:
             step(to_device(hb, dev))
-        state["loss_host"] = float(state["loss"].item())     # D2H read of the step's result
+        state["loss_host"] = float(state["out"]["loss"].item())     # D2H read of the step's result
 
     e2e_step()
     ms_e2e = timed_region(e2e_step, args.steps)

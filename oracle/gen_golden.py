@@ -10,7 +10,9 @@ Every output array comes from reference classes:
   packnet_sfm.networks.layers.packnet.layers01.{PackLayerConv3d,UnpackLayerConv3d,Conv2D,ResidualConv}
   packnet_sfm.networks.depth.PackNet01.PackNet01
 Inputs and weights are regenerated from seeds (packnet_sfm_b200/synthetic.py, oracle/packnet_oracle.py);
-the inputs are stored too so an RNG change cannot silently invalidate a fixture.
+the inputs are stored too (the block inputs as their seed and shape, the large ones as a checksum) so an RNG
+change cannot silently invalidate a fixture.  No fixture file exceeds 1 MB: large gradients are stored as a
+seeded sample plus their norm, the larger depth maps of the full-size cases at a pixel stride.
 """
 import os
 import sys
@@ -83,35 +85,109 @@ def _load(module, sd):
     return module
 
 
+def seeded_input(arrays, key, shape, seed):
+    """A uniform(-0.5, 0.5) input, stored as its seed and shape (tests/conftest.py:load_golden regenerates it)."""
+    arrays[key + "/seed"] = np.int64(seed)
+    arrays[key + "/shape"] = np.array(shape, dtype=np.int64)
+    return torch.rand(shape, generator=torch.Generator().manual_seed(seed)) - 0.5
+
+
+def store_sampled(arrays, key, t, n=4096, seed=0):
+    """A tensor of more than 8n elements is stored as n seeded random elements (`key/idx` flat positions, `key/samp`) and
+    the whole tensor's float64 norm (`key/norm`); keeps every fixture file under 1 MB."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= 8 * n:
+        arrays[key] = t.detach()
+        return
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(seed))[:n].sort().values
+    arrays[key + "/idx"] = idx.to(torch.int32)
+    arrays[key + "/samp"] = flat[idx]
+    arrays[key + "/norm"] = np.float64(flat.double().norm().item())
+
+
 def block_cases():
     arrays = {}
-    g = torch.Generator().manual_seed(5)
 
-    def run(tag, module, sd, x):
+    def run(i, tag, module, sd, shape):
         _load(module, sd)
-        x = x.clone().requires_grad_(True)
+        x = seeded_input(arrays, tag + "_x", shape, 50 + 2 * i).requires_grad_(True)
         y = module(x)
-        gy = torch.rand(y.shape, generator=g) - 0.5
+        gy = seeded_input(arrays, tag + "_gy", tuple(y.shape), 51 + 2 * i)
         y.backward(gy)
-        arrays[tag + "_x"] = x.detach()
         arrays[tag + "_y"] = y.detach()
-        arrays[tag + "_gy"] = gy
         arrays[tag + "_gx"] = x.grad
         for k, p in module.named_parameters():
-            arrays[tag + "_g_" + k] = p.grad
+            store_sampled(arrays, tag + "_g_" + k, p.grad, seed=i)
 
-    run("pack_k3", L.PackLayerConv3d(32, 3), PO.block_state_dict("pack", 32, k=3, seed=21),
-        torch.rand(2, 32, 16, 24, generator=g) - 0.5)
-    run("pack_k5", L.PackLayerConv3d(16, 5), PO.block_state_dict("pack", 16, k=5, seed=22),
-        torch.rand(1, 16, 12, 40, generator=g) - 0.5)
-    run("unpack", L.UnpackLayerConv3d(64, 32, 3), PO.block_state_dict("unpack", 64, 32, 3, seed=23),
-        torch.rand(2, 64, 6, 20, generator=g) - 0.5)
-    run("conv2d_k7", L.Conv2D(32, 32, 7, 1), PO.block_state_dict("conv2d", 32, 32, 7, seed=24),
-        torch.rand(1, 32, 12, 20, generator=g) - 0.5)
-    run("residual", L.ResidualConv(32, 64, 1), PO.block_state_dict("residual", 32, 64, seed=25),
-        torch.rand(2, 32, 8, 12, generator=g) - 0.5)
-    np.savez_compressed(os.path.join(OUT, "blocks.npz"), **{k: v.numpy() for k, v in arrays.items()})
+    run(0, "pack_k3", L.PackLayerConv3d(32, 3), PO.block_state_dict("pack", 32, k=3, seed=21), (2, 32, 16, 24))
+    run(1, "pack_k5", L.PackLayerConv3d(16, 5), PO.block_state_dict("pack", 16, k=5, seed=22), (1, 16, 12, 40))
+    run(2, "unpack", L.UnpackLayerConv3d(64, 32, 3), PO.block_state_dict("unpack", 64, 32, 3, seed=23), (2, 64, 6, 20))
+    run(3, "conv2d_k7", L.Conv2D(32, 32, 7, 1), PO.block_state_dict("conv2d", 32, 32, 7, seed=24), (1, 32, 12, 20))
+    run(4, "residual", L.ResidualConv(32, 64, 1), PO.block_state_dict("residual", 32, 64, seed=25), (2, 32, 8, 12))
+    np.savez_compressed(os.path.join(OUT, "blocks.npz"),
+                        **{k: v.numpy() if torch.is_tensor(v) else v for k, v in arrays.items()})
     print("blocks", len(arrays))
+
+
+def restatement_case():
+    """The reference's PackNet01 as a module: its state-dict names and shapes, and its depth maps for the oracle's default
+    weights (Xavier-uniform convolutions, zero biases, GroupNorm affine (1, 0))."""
+    net = PackNet01(version="1A").train()
+    arrays = {"keys": np.array(list(net.state_dict()))}
+    for k, v in net.state_dict().items():
+        arrays["shape/" + k] = np.array(v.shape, dtype=np.int64)
+    _load(net, PO.packnet01_state_dict())
+    x = synthetic.make_frames(1, 64, 96, seed=3)["rgb"]
+    with torch.no_grad():
+        out = net(x)["inv_depths"]
+    arrays["rgb"] = x.numpy()
+    for i, d in enumerate(out):
+        arrays["disp%d" % (i + 1)] = d.numpy()
+    np.savez_compressed(os.path.join(OUT, "packnet01_restatement_64x96.npz"), **arrays)
+    print("packnet01_restatement", len(arrays["keys"]), float(out[0].mean()))
+
+
+def loss_restatement_case():
+    """The reference's MultiViewPhotometricLoss with the training defaults on four full-resolution maps."""
+    B, H, W = 2, 24, 48
+    fr = synthetic.make_frames(B, H, W, seed=5)
+    inv = synthetic.make_inv_depths(B, H, W, seed=6)
+    mats = [pose_from_vec(synthetic.make_pose_vecs(B, seed=7)[:, j]) for j in range(2)]
+    loss_fn = MultiViewPhotometricLoss(num_scales=4, ssim_loss_weight=0.85, smooth_loss_weight=0.001,
+                                       photometric_reduce_op="min", clip_loss=0.0, automask_loss=True)
+    K = fr["intrinsics"]
+    out = loss_fn(fr["rgb"], fr["rgb_context"], inv, K, K, [Pose(m.clone()) for m in mats])
+    arrays = {"rgb": fr["rgb"], "ctx0": fr["rgb_context"][0], "ctx1": fr["rgb_context"][1], "K": K,
+              "loss": out["loss"]}
+    arrays.update({"inv%d" % i: d for i, d in enumerate(inv)})
+    arrays.update({"pose%d" % j: m for j, m in enumerate(mats)})
+    np.savez_compressed(os.path.join(OUT, "loss_restatement_2x24x48.npz"), **{k: v.detach().numpy() for k, v in arrays.items()})
+    print("loss_restatement", float(out["loss"]))
+
+
+def selfsup_flip_case():
+    """The reference's own SelfSupModel.forward (left-right flip forced, maps upsampled) with its PackNet01, PoseNet and
+    loss: loss, metrics and the four depth maps of one training-mode forward."""
+    from oracle.step_oracle import posenet_state_dict
+    from packnet_sfm.models.SelfSupModel import SelfSupModel
+    from packnet_sfm.networks.pose.PoseNet import PoseNet
+    H, W = 32, 64
+    fr = synthetic.make_frames(1, H, W, seed=3)
+    batch = {"rgb": fr["rgb"], "rgb_context": fr["rgb_context"], "rgb_original": fr["rgb"],
+             "rgb_context_original": fr["rgb_context"], "intrinsics": fr["intrinsics"]}
+    depth = _load(PackNet01(version="1A"), PO.packnet01_state_dict(seed=42, randomize_affine=True))
+    pose = _load(PoseNet(nb_ref_imgs=2, rotation_mode="euler"), posenet_state_dict(43))
+    model = SelfSupModel(depth_net=depth, pose_net=pose, num_scales=4, ssim_loss_weight=0.85, smooth_loss_weight=0.001,
+                         photometric_reduce_op="min", clip_loss=0.0, automask_loss=True, rotation_mode="euler",
+                         flip_lr_prob=1.0, upsample_depth_maps=True).train()
+    with torch.no_grad():
+        out = model(batch)
+    arrays = {"rgb": fr["rgb"], "ctx0": fr["rgb_context"][0], "ctx1": fr["rgb_context"][1], "K": fr["intrinsics"],
+              "loss": out["loss"], "photometric_loss": out["metrics"]["photometric_loss"],
+              "smoothness_loss": out["metrics"]["smoothness_loss"]}
+    arrays.update({"inv%d" % i: d for i, d in enumerate(out["inv_depths"])})
+    np.savez_compressed(os.path.join(OUT, "selfsup_flip_1x32x64.npz"), **{k: v.numpy() for k, v in arrays.items()})
+    print("selfsup_flip", float(out["loss"]))
 
 
 def packnet_case():
@@ -145,9 +221,9 @@ def _grad_samples(named_grads, arrays, prefix, n=64):
         arrays[prefix + "samp/" + k] = flat[idx].numpy()
 
 
-def packnet_baseline_case(B=4, H=192, W=640, name="packnet01_192x640_b4", disp1_stride=1):
+def packnet_baseline_case(B=4, H=192, W=640, name="packnet01_192x640_b4", strides=(2, 2, 1, 1)):
     """PackNet01 at BASELINE configs[1] (B=4, 192x640): the engine paths that the 64x96 fixture cannot reach (persistent
-    tile loop, batch folding, split-K thresholds).  Depth maps in full (fp32), the gradient of sum_i <disp_i, gy_i> for a
+    tile loop, batch folding, split-K thresholds).  Depth maps (fp32; map i at every strides[i]-th pixel), the gradient of sum_i <disp_i, gy_i> for a
     seeded gy as per-parameter norms + strided samples.  The input is regenerated from its seed by the test; a checksum
     guards against an RNG change."""
     sd = PO.packnet01_state_dict(seed=42, randomize_affine=True)
@@ -163,9 +239,9 @@ def packnet_baseline_case(B=4, H=192, W=640, name="packnet01_192x640_b4", disp1_
     for i, d in enumerate(out):
         gy = torch.rand(d.shape, generator=g) - 0.5
         obj = obj + (d * gy).sum()
-        # the full-resolution map of the large fixtures is stored at every second pixel (fixture size)
-        arrays["disp%d" % (i + 1)] = d.detach()[..., ::disp1_stride, ::disp1_stride].numpy() if i == 0 else d.detach().numpy()
-    arrays["disp1_stride"] = np.int64(disp1_stride)
+        # the larger maps are stored at every strides[i]-th pixel in both directions (fixture size)
+        arrays["disp%d" % (i + 1)] = d.detach()[..., ::strides[i], ::strides[i]].numpy()
+        arrays["disp%d_stride" % (i + 1)] = np.int64(strides[i])
     obj.backward()
     _grad_samples([(k, p.grad) for k, p in net.named_parameters()], arrays, "g")
     np.savez_compressed(os.path.join(OUT, name + ".npz"), **arrays)
@@ -174,7 +250,7 @@ def packnet_baseline_case(B=4, H=192, W=640, name="packnet01_192x640_b4", disp1_
 
 def packnet_config3_case():
     """BASELINE configs[2]'s per-GPU shape: B=2, 384x1280."""
-    packnet_baseline_case(B=2, H=384, W=1280, name="packnet01_384x1280_b2", disp1_stride=2)
+    packnet_baseline_case(B=2, H=384, W=1280, name="packnet01_384x1280_b2", strides=(4, 2, 1, 1))
 
 
 def step_case(B=2, H=64, W=96, name="step_2x64x96"):
@@ -242,6 +318,10 @@ if __name__ == "__main__":
     loss_case("loss_bigmotion", 2, 32, 64, True, big_motion=True)
     loss_case("loss_progressive", 1, 32, 64, False, progressive_scaling=0.2)
     block_cases()
+    restatement_case()
+    loss_restatement_case()
+    selfsup_flip_case()
     packnet_case()
     step_case()
     packnet_baseline_case()
+    packnet_config3_case()

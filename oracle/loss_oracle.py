@@ -12,8 +12,8 @@ Restates, with file:line citations into /root/reference/packnet_sfm:
   losses/loss_base.py:9-48         ProgressiveScaling
   models/model_utils.py:152-180    upsample_output (nearest)
 
-Pinned against the live reference by tests/test_oracle_vs_reference.py (build container) and against
-tests/golden/loss_*.npz (generated from the live reference by oracle/gen_golden.py) everywhere.
+Pinned against tests/golden/loss_*.npz, generated from the live reference by oracle/gen_golden.py
+(tests/test_oracle_vs_reference.py, tests/test_oracle_golden.py).
 
 `warp_tap_indices` is the integer oracle for the "warp pixel indices bit-exact" bar: it spells out the
 reference's fp32 operation chain one rounding at a time in numpy (numpy never contracts a*b+c into an

@@ -5,8 +5,8 @@ Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl refere
 
 Every function cites the reference file:line it restates (paths relative to /root/reference).
 The restatement is pinned two ways (SURVEY.md §8c -- the reference ships no tests or golden vectors):
-  * tests/test_oracle_vs_reference.py runs it against the live, unmodified reference in the build
-    container (skipped where /root/reference is absent), and
+  * tests/test_oracle_vs_reference.py holds it to the unmodified reference module's state-dict names,
+    shapes and depth maps (stored by oracle/gen_golden.py), and
   * tests/golden/*.npz hold input/output vectors generated from the live reference by
     oracle/gen_golden.py; tests/test_oracle_golden.py checks the restatement against them everywhere.
 

@@ -1,8 +1,8 @@
 """Import shims so the UNMODIFIED reference (/root/reference) runs on CPU in the build container.
 
 TEST INFRASTRUCTURE ONLY.  Nothing in the product path (packnet_sfm_b200/) may import this.
-It is used by oracle/gen_golden.py (fixture generation, build container only) and by the
-`ref`-marked validation tests; /root/reference does not exist on the GPU box.
+It is used by oracle/gen_golden.py, which generates the fixtures under tests/golden/ where the
+reference tree is present; the tests read only those fixtures.
 
 Shims (none touches arithmetic; SURVEY.md §8c):
   * stub `yacs` / `yacs.config.CfgNode`      (packnet_sfm/utils/types.py:3,41-43 — isinstance helper only)

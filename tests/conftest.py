@@ -44,8 +44,30 @@ def pytest_collection_modifyitems(config, items):
 
 
 def load_golden(name):
+    """Fixture arrays by name; a uniform(-0.5, 0.5) input stored as `key/seed` + `key/shape` (oracle/gen_golden.py:
+    seeded_input) comes back regenerated under `key`."""
     z = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
-    return {k: (torch.from_numpy(z[k]) if z[k].dtype.kind == "f" else z[k]) for k in z.files}
+    out = {k: (torch.from_numpy(z[k]) if z[k].dtype.kind == "f" else z[k]) for k in z.files}
+    for k in [k[:-len("/seed")] for k in z.files if k.endswith("/seed")]:
+        g = torch.Generator().manual_seed(int(z[k + "/seed"]))
+        out[k] = torch.rand(tuple(int(s) for s in z[k + "/shape"]), generator=g) - 0.5
+    return out
+
+
+def assert_golden_close(got, z, key, rel, floor):
+    """||got - golden|| <= rel * ||golden|| + floor * sqrt(numel) over the elements the fixture stores for `key`: the whole
+    tensor, or the seeded sample of a large one (oracle/gen_golden.py:store_sampled), whose whole-tensor norm must then
+    lie within the same bound of the stored norm."""
+    got = got.detach().cpu().double()
+    if key in z:
+        ref = z[key].double()
+    else:
+        norm = float(z[key + "/norm"])
+        bound = rel * norm + floor * got.numel() ** 0.5
+        assert abs(float(got.norm()) - norm) <= bound, (key, float(got.norm()), norm)
+        got, ref = got.reshape(-1)[torch.from_numpy(z[key + "/idx"]).long()], z[key + "/samp"].double()
+    err = float((got - ref).norm())
+    assert err <= rel * float(ref.norm()) + floor * ref.numel() ** 0.5, (key, err)
 
 
 @pytest.fixture

@@ -9,7 +9,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from conftest import load_golden, rel_l2
+from conftest import assert_golden_close, load_golden, rel_l2
 from oracle import packnet_oracle as PO
 
 pytestmark = pytest.mark.gpu
@@ -130,9 +130,7 @@ def test_folded_pack_block_matches_reference_golden(tag, cin, k, seed):
     assert rel_l2(nchw(y).cpu(), z[tag + "_y"]) < 1e-4, rel_l2(nchw(y).cpu(), z[tag + "_y"])
     assert rel_l2(nchw(x.grad).cpu(), z[tag + "_gx"]) < 1e-3
     for name, p in mod.named_parameters():
-        ref = z[tag + "_g_" + name]
-        err = float((p.grad.cpu().double() - ref.double()).norm())
-        assert err <= 1e-3 * float(ref.double().norm()) + 5e-5 * ref.numel() ** 0.5, (tag, name, err)
+        assert_golden_close(p.grad, z, tag + "_g_" + name, 1e-3, 5e-5)
 
 
 def test_packnet01_with_folded_pack_layers_matches_reference_golden():

@@ -5,7 +5,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from conftest import load_golden, rel_l2
+from conftest import assert_golden_close, load_golden, rel_l2
 from oracle import packnet_oracle as PO
 
 pytestmark = pytest.mark.gpu
@@ -181,6 +181,4 @@ def test_blocks_match_reference_golden(tag, make, sd):
     assert rel_l2(nchw(y).cpu(), z[tag + "_y"]) < 1e-4, rel_l2(nchw(y).cpu(), z[tag + "_y"])
     assert rel_l2(nchw(x.grad).cpu(), z[tag + "_gx"]) < 1e-3
     for k, p in mod.named_parameters():
-        ref = z[tag + "_g_" + k]
-        err = float((p.grad.cpu().double() - ref.double()).norm())
-        assert err <= 1e-3 * float(ref.double().norm()) + 5e-5 * ref.numel() ** 0.5, (tag, k, err)
+        assert_golden_close(p.grad, z, tag + "_g_" + k, 1e-3, 5e-5)

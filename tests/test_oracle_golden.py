@@ -8,7 +8,7 @@ import torch
 
 from oracle import loss_oracle as LO
 from oracle import packnet_oracle as PO
-from conftest import load_golden, rel_l2
+from conftest import assert_golden_close, load_golden, rel_l2
 
 LOSS_CASES = ["loss_fullres", "loss_multires", "loss_mean_noautomask", "loss_bigmotion", "loss_progressive"]
 
@@ -95,9 +95,7 @@ def test_pack_unpack_oracle_matches_reference_golden():
         for k, p in sd.items():
             # a conv bias feeding GroupNorm has a mathematically zero gradient: only rounding noise
             # (~1e-6) is left, so use an absolute floor next to the relative bound
-            ref = z[tag + "_g_" + k]
-            err = float((p.grad.double() - ref.double()).norm())
-            assert err <= 1e-5 * float(ref.double().norm()) + 2e-5 * ref.numel() ** 0.5, (tag, k)
+            assert_golden_close(p.grad, z, tag + "_g_" + k, 1e-5, 2e-5)
 
 
 def test_packnet01_oracle_matches_reference_golden():

@@ -1,45 +1,33 @@
-"""Build-container only (marker `ref`): the oracle restatement against the LIVE unmodified reference."""
-import pytest
+"""CPU: the oracle restatement against what the unmodified reference's own module and loss class computed
+(oracle/gen_golden.py: restatement_case, loss_restatement_case)."""
 import torch
 
-from conftest import rel_l2
-
-pytestmark = pytest.mark.ref
+from conftest import load_golden
 
 
-def test_packnet01_restatement_is_bit_identical_to_reference_module():
-    from oracle import ref_shims
-    ref_shims.install()
-    from packnet_sfm.networks.depth.PackNet01 import PackNet01
+def test_packnet01_restatement_matches_reference_module():
+    """Same parameter names, order and shapes as the reference's PackNet01, and its depth maps for the same weights.  The
+    oracle runs the reference's ops in the reference's order, so with the CPU convolution kernels that produced the fixture
+    the maps are bit-identical; a host whose oneDNN picks other kernels (AVX2 instead of AVX-512) sums in another order,
+    which moves them by up to 4e-5 relative."""
     from oracle import packnet_oracle as PO
-    from packnet_sfm_b200 import synthetic
-    torch.manual_seed(0)
-    net = PackNet01(version="1A").train()
-    sd = {k: v.detach() for k, v in net.state_dict().items()}
-    sd2 = PO.packnet01_state_dict()
-    assert set(sd) == set(sd2) and all(sd[k].shape == sd2[k].shape for k in sd)
-    x = synthetic.make_frames(1, 64, 96, seed=3)["rgb"]
+    z = load_golden("packnet01_restatement_64x96")
+    sd = PO.packnet01_state_dict()
+    assert list(sd) == list(z["keys"])
+    assert all(tuple(sd[k].shape) == tuple(int(s) for s in z["shape/" + k]) for k in sd)
     with torch.no_grad():
-        ref = net(x)["inv_depths"]
-        mine = PO.packnet01_forward(x, sd)
-    for a, b in zip(ref, mine):
-        assert torch.equal(a, b)
+        mine = PO.packnet01_forward(z["rgb"], sd)
+    for i, a in enumerate(mine):
+        b = z["disp%d" % (i + 1)]
+        assert a.shape == b.shape
+        assert float(((a - b).abs() / b.abs()).max()) < 1e-4, i
 
 
 def test_loss_restatement_matches_reference_class():
-    from oracle import ref_shims
-    ref_shims.install()
-    from packnet_sfm.losses.multiview_photometric_loss import MultiViewPhotometricLoss
-    from packnet_sfm.geometry.pose import Pose
+    """Same ops in the same order as the reference's MultiViewPhotometricLoss: bit-identical on the host that produced the
+    fixture; 1e-6 leaves room for another host's CPU kernels (as tests/test_oracle_golden.py)."""
     from oracle import loss_oracle as LO
-    from packnet_sfm_b200 import synthetic
-    B, H, W = 2, 24, 48
-    fr = synthetic.make_frames(B, H, W, seed=5)
-    inv = synthetic.make_inv_depths(B, H, W, seed=6)
-    mats = [LO.pose_from_vec(synthetic.make_pose_vecs(B, seed=7)[:, j]) for j in range(2)]
-    ref = MultiViewPhotometricLoss(num_scales=4, ssim_loss_weight=0.85, smooth_loss_weight=0.001,
-                                   photometric_reduce_op="min", clip_loss=0.0, automask_loss=True)
-    K = fr["intrinsics"]
-    a = ref(fr["rgb"], fr["rgb_context"], inv, K, K, [Pose(m.clone()) for m in mats])
-    b = LO.multiview_photometric_loss(fr["rgb"], fr["rgb_context"], inv, K, K, mats)
-    assert float(a["loss"]) == float(b["loss"])
+    z = load_golden("loss_restatement_2x24x48")
+    inv = [z["inv%d" % i] for i in range(4)]
+    out = LO.multiview_photometric_loss(z["rgb"], [z["ctx0"], z["ctx1"]], inv, z["K"], z["K"], [z["pose0"], z["pose1"]])
+    assert abs(float(out["loss"]) - float(z["loss"])) <= 1e-6 * abs(float(z["loss"]))

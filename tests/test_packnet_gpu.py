@@ -108,11 +108,11 @@ def strided_index(numel, n):
 
 @pytest.mark.parametrize("fixture,B,H,W", [("packnet01_192x640_b4", 4, 192, 640), ("packnet01_384x1280_b2", 2, 384, 1280)])
 def test_packnet01_baseline_config_matches_reference_golden(pack_path, fixture, B, H, W):
-    """BASELINE configs[1] (B=4, 192x640) and the per-GPU shape of configs[2] (B=2, 384x1280; full-resolution map stored at
-    every second pixel): the engine paths the 64x96 fixture does not reach -- persistent tile loop with
-    hundreds of work items, batch folding on the small maps, the split-K thresholds -- against the LIVE reference's depth
-    maps (tests/golden/packnet01_192x640_b4.npz: fp32 maps in full, gradients of sum_i <disp_i, gy_i> as per-parameter
-    norms + 64 strided samples).  Bar: depth 1e-3 max-relative (north_star); gradients 2e-3 of the tensor's norm."""
+    """BASELINE configs[1] (B=4, 192x640) and the per-GPU shape of configs[2] (B=2, 384x1280): the engine paths the 64x96
+    fixture does not reach -- persistent tile loop with hundreds of work items, batch folding on the small maps, the split-K
+    thresholds -- against the reference's depth maps (tests/golden/packnet01_192x640_b4.npz: fp32 maps, the larger ones at
+    every disp<i>_stride-th pixel in both directions; gradients of sum_i <disp_i, gy_i> as per-parameter norms + 64
+    strided samples).  Bar: depth 1e-3 max-relative (north_star); gradients 2e-3 of the tensor's norm."""
     from packnet_sfm_b200 import synthetic
     z = load_golden(fixture)
     x = synthetic.make_frames(B, H, W, seed=int(z["seed_rgb"]))["rgb"]
@@ -123,12 +123,10 @@ def test_packnet01_baseline_config_matches_reference_golden(pack_path, fixture, 
     g = torch.Generator().manual_seed(int(z["seed_gy"]))
     gys = [torch.rand(d.shape, generator=g) - 0.5 for d in out]
     worst = 0.0
-    stride1 = int(z["disp1_stride"]) if "disp1_stride" in z else 1
     for i, d in enumerate(out):
         ref = z["disp%d" % (i + 1)]
-        got = d.detach().cpu()
-        if i == 0 and stride1 > 1:
-            got = got[..., ::stride1, ::stride1]
+        stride = int(z["disp%d_stride" % (i + 1)])
+        got = d.detach().cpu()[..., ::stride, ::stride]
         assert got.shape == ref.shape
         rel = ((got - ref).abs() / ref.abs()).max().item()
         worst = max(worst, rel)
